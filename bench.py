@@ -5,6 +5,7 @@ clouds -- BASELINE.json `metric`, configs[1].
     python bench.py --gpus N --steps K --warmup W                 (N>1: launched under torchrun, one rank per GPU)
     python bench.py --config {second,pillars,cbgs} ...            (BASELINE configs[1] / [2] / [3] at their stated sizes)
     python bench.py --impl reference ...                          (the reference path on the host cores)
+    python bench.py --dump-outputs DIR ...                        (also write the last timed step's detections to DIR)
 
 One step = one pass of the whole hot path (voxelize -> reader -> sparse middle encoder -> RPN -> heads -> decode /
 top-k / rotated NMS) over one batch of clouds per GPU.  The ranks' detections are exchanged with ONE all-gather after
@@ -49,7 +50,11 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying a CUDA graph")
     ap.add_argument("--gather-every", type=int, default=0, help="all-gather the detections every G steps (0: once, after the last step)")
     ap.add_argument("--no-nms-c5", action="store_true", help="skip the 100k-box NMS stress (BASELINE configs[4]) leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the detections of the last one as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.wl = WORKLOADS[args.config]
     if args.batch is None:
         args.batch = args.wl["batch"]
@@ -246,8 +251,10 @@ def run_reference(args, rank, world):
         cpu.forward([clouds[(i + j) % N_CLOUD_POOL] for j in range(sample)])
     t0 = time.perf_counter()
     for i in range(args.steps):
-        cpu.forward([clouds[(i * sample + j) % N_CLOUD_POOL] for j in range(sample)])
+        dets = cpu.forward([clouds[(i * sample + j) % N_CLOUD_POOL] for j in range(sample)])
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dets)
     value = args.steps * sample / dt
     line = {
         "impl": "reference", "metric": "point-clouds/sec SECOND SpMiddleFHD @20k pts", "value": value,
@@ -290,6 +297,27 @@ def _claim_stdout():
 def _emit(line):
     sys.stdout.flush()
     os.write(_REAL_STDOUT if _REAL_STDOUT is not None else 1, (json.dumps(line) + "\n").encode())
+
+
+DUMP_BUDGET = 64 << 20
+
+
+def dump_outputs(out_dir, dets):
+    """The detections a caller receives for each cloud of one step, as cloud<j>_{box3d_lidar,scores,label_preds}.npy
+    (float32; class ids are exact in float32).  Clouds and weights are seeded, so two builds run with the same arguments
+    can be compared file for file.  Clouds past DUMP_BUDGET bytes are left out (a fixed prefix of the batch)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for j, det in enumerate(dets):
+        arrays = {k: det[k].detach().cpu().numpy().astype(np.float32) for k in ("box3d_lidar", "scores", "label_preds")}
+        size = sum(a.nbytes for a in arrays.values())
+        if total + size > DUMP_BUDGET:
+            print("[bench] --dump-outputs: clouds %d.. left out (%d MiB budget)" % (j, DUMP_BUDGET >> 20), file=sys.stderr)
+            break
+        total += size
+        for k, a in arrays.items():
+            np.save(os.path.join(out_dir, "cloud%d_%s.npy" % (j, k)), a)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -488,6 +516,8 @@ def main():
     sampler.mark()                      # clocks are sampled from here to the end of the per-kernel pass (same load)
     ms = timed(step_device, args.steps, False)
     ms_e2e = timed(step_e2e, args.steps, True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pipe.unpack(state["out_pinned"]))       # the last step_e2e, already on the host
 
     # ---- per-stage pass: eager launches of the SAME kernels, CUDA events around every det3d_b200 call on the
     #      launching stream (voxelize / rulebook / sparse convs / dense convs / predict): launch count + rooflines ----

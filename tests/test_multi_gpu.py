@@ -27,7 +27,7 @@ def _run(world, config, clouds, port):
 def test_cbgs_32_clouds_sharded_over_all_gpus():
     n = torch.cuda.device_count()
     if n < 2:
-        pytest.skip("needs >= 2 GPUs (run under gpurun --gpus N)")
+        pytest.skip("needs >= 2 GPUs")
     world = max(w for w in (2, 4, 8) if w <= n)
     r = _run(world, "cbgs", 32, 29671)
     assert r["world"] == world and r["clouds"] == 32 and r["gathered_equals_single_rank"] is True

@@ -1,9 +1,9 @@
 """Pins the voxelizer oracle (C restatement + numpy restatement) to the reference numba
-function through the committed golden fixtures (tests/golden/make_golden.py)."""
+function through the committed golden fixtures (tests/golden/make_golden.py, make_golden_reference.py)."""
 import numpy as np
 import pytest
 
-from conftest import golden_voxel_cases, has_reference, load_golden
+from conftest import array_digest, golden_voxel_cases, load_golden
 from oracle import voxel as ovoxel
 
 
@@ -45,36 +45,27 @@ def test_dense_map_scratch_is_restored():
     assert all(np.array_equal(x, y) for x, y in zip(a, b))
 
 
-@pytest.mark.skipif(not has_reference(), reason="reference checkout not present")
-def test_c_oracle_matches_live_reference_on_fresh_seeds():
-    import importlib.util
-
-    spec = importlib.util.spec_from_file_location("ref_pc_ops", "/root/reference/det3d/ops/point_cloud/point_cloud_ops.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+def _fresh_seed_clouds():
+    """(points, voxel_size, range, max_points, max_voxels): three seeded KITTI-grid clouds, ~1 m beyond the range."""
     rng = np.random.default_rng(123)
     vs, pcr = np.float32([0.05, 0.05, 0.1]), np.float32([0, -40, -3, 70.4, 40, 1])
+    cases = []
     for seed in range(3):
         n = int(rng.integers(100, 5000))
         pts = np.stack([rng.uniform(-1, 71, n), rng.uniform(-41, 41, n), rng.uniform(-3.2, 1.2, n), rng.uniform(0, 1, n)], 1).astype(np.float32)
-        a = ref.points_to_voxel(pts, vs, pcr, 5, True, 600 + 700 * seed)
-        b = ovoxel.points_to_voxel(pts, vs, pcr, 5, True, 600 + 700 * seed)
-        assert all(np.array_equal(x, y) for x, y in zip(a, b))
+        cases.append((pts, vs, pcr, 5, 600 + 700 * seed))
+    return cases
 
 
-def test_c_oracle_equals_aot_reference_kernel_on_random_inputs():
-    """Beyond the committed goldens: when oracle/_ref holds the reference's own numba kernel compiled ahead of time
-    (oracle/build.py, built where /root/reference exists), the C restatement must reproduce it bit for bit on fresh
-    seeded clouds -- boundary-snapped points, overflow `break`, ndim 3/4/5, an empty cloud."""
-    from oracle import voxel, voxel_ref
-
-    if not voxel_ref.available():
-        pytest.skip("oracle/_ref/ref_voxel_aot*.so not built (reference checkout absent at build time)")
+def _random_clouds():
+    """(points, voxel_size, range, max_points, max_voxels): boundary-snapped points, the max_voxels `break`, ndim 3/4/5,
+    an empty cloud."""
     rng = np.random.default_rng(123)
     cases = [([0.05, 0.05, 0.1], [0, -40.0, -3.0, 70.4, 40.0, 1.0], 5, 20000, 4, 30000),
              ([0.16, 0.16, 4.0], [0, -39.68, -3, 69.12, 39.68, 1], 100, 1200, 4, 9000),      # hits the max_voxels break
              ([0.1, 0.1, 0.2], [-51.2, -51.2, -5.0, 51.2, 51.2, 3.0], 10, 60000, 5, 20000),
              ([0.05, 0.05, 0.1], [0, -40.0, -3.0, 70.4, 40.0, 1.0], 5, 20000, 3, 0)]
+    out = []
     for vs, pcr, max_pts, max_vox, ndim, n in cases:
         lo, hi = np.asarray(pcr[:3], np.float32), np.asarray(pcr[3:], np.float32)
         span = (hi - lo + 2.0)[[0, 1, 2] + [0] * (ndim - 3)]
@@ -84,7 +75,33 @@ def test_c_oracle_equals_aot_reference_kernel_on_random_inputs():
             snap = rng.random(n) < 0.3            # exact multiples of the voxel size: fp32 division edge cases
             cell = np.floor((pts[snap, :3] - lo) / np.asarray(vs, np.float32))
             pts[snap, :3] = lo + cell * np.asarray(vs, np.float32)
-        want = voxel_ref.points_to_voxel(pts, vs, pcr, max_pts, True, max_vox)
-        got = voxel.points_to_voxel(pts, vs, pcr, max_pts, True, max_vox)
-        for a, b in zip(got, want):
-            assert a.dtype == b.dtype and np.array_equal(a, b)
+        out.append((pts, vs, pcr, max_pts, max_vox))
+    return out
+
+
+def _assert_reference_output(g, key, pts, got):
+    """`got` (voxels, coors, num_points) against the reference's output stored under `key`: the voxel count, a fixed
+    sample of voxels (readable on failure), then every array bit for bit through its digest."""
+    assert array_digest(pts) == str(g[key + "_points"]), "input cloud changed: regenerate the golden"
+    idx = g[key + "_sample"]
+    for name, a in zip(("voxels", "coors", "num_points"), got):
+        assert a.shape[0] == int(g[key + "_count"]), (key, name)
+        assert np.array_equal(a[idx], g[key + "_" + name + "_sample"]), (key, name)
+        assert array_digest(a) == str(g[key + "_" + name]), (key, name)
+
+
+def test_c_oracle_matches_live_reference_on_fresh_seeds():
+    """The reference's numba `points_to_voxel` (point_cloud_ops.py:112-184) on three seeded clouds; its outputs are
+    stored in tests/golden/ref_voxel_fresh_seeds.npz (tests/golden/make_golden_reference.py)."""
+    g = load_golden("ref_voxel_fresh_seeds")
+    for i, (pts, vs, pcr, max_pts, max_vox) in enumerate(_fresh_seed_clouds()):
+        _assert_reference_output(g, "s%d" % i, pts, ovoxel.points_to_voxel(pts, vs, pcr, max_pts, True, max_vox))
+
+
+def test_c_oracle_equals_aot_reference_kernel_on_random_inputs():
+    """Beyond the committed goldens: the C restatement must reproduce the reference's own numba kernel bit for bit on
+    seeded clouds -- boundary-snapped points, overflow `break`, ndim 3/4/5, an empty cloud.  The reference outputs are
+    stored in tests/golden/ref_voxel_random.npz (tests/golden/make_golden_reference.py)."""
+    g = load_golden("ref_voxel_random")
+    for i, (pts, vs, pcr, max_pts, max_vox) in enumerate(_random_clouds()):
+        _assert_reference_output(g, "c%d" % i, pts, ovoxel.points_to_voxel(pts, vs, pcr, max_pts, True, max_vox))

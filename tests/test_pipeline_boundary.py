@@ -1,14 +1,13 @@
 """The reference's dataset-side boundary (SURVEY 2.1 #16, 8a4): `Voxelization`, `AssignTarget`, `Reformat`, `Compose`
 (det3d/datasets/pipelines/) and `collate_kitti` (det3d/torchie/parallel/collate.py:90-150) under their own names."""
-import ast
-import collections
+import json
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import REFERENCE, ROOT, has_reference
+from conftest import ROOT, load_golden, reference_config
 
 STOCK = [
     "examples/second/configs/kitti_car_vfev3_spmiddlefhd_rpn1_mghead_syncbn.py",
@@ -17,14 +16,12 @@ STOCK = [
 ]
 
 
-@pytest.mark.skipif(not has_reference(), reason="reference checkout not present")
 @pytest.mark.parametrize("rel", STOCK)
 def test_stock_test_pipeline_builds(rel):
     """cfg.test_pipeline of an UNMODIFIED reference config builds through PIPELINES (every step is registered)."""
     from det3d.datasets.pipelines import Compose
-    from det3d.torchie import Config
 
-    cfg = Config.fromfile(os.path.join(REFERENCE, rel))
+    cfg = reference_config(rel)
     pipe = Compose(cfg.test_pipeline)
     names = [type(t).__name__ for t in pipe.transforms]
     assert names == ["LoadPointCloudFromFile", "LoadPointCloudAnnotations", "Preprocess", "Voxelization", "AssignTarget",
@@ -63,13 +60,22 @@ def _sample(i, n_vox, max_pts=5, ndim=4, n_anchor=12):
     )
 
 
-def _reference_collate():
-    """The reference function itself, lifted out of its module (whose package imports do not resolve here)."""
-    src = open(os.path.join(REFERENCE, "det3d/torchie/parallel/collate.py")).read()
-    fn = next(n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "collate_kitti")
-    ns = dict(np=np, torch=torch, collections=collections, defaultdict=collections.defaultdict)
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), "collate.py", "exec"), ns)
-    return ns["collate_kitti"]
+def _reference_collate_result():
+    """The reference `collate_kitti` on the batch of test_collate_kitti_equals_reference_function, stored by
+    tests/golden/make_golden_reference.py: a JSON skeleton whose tensors and arrays are the other entries."""
+    g = load_golden("ref_collate_kitti")
+
+    def build(node):
+        kind, v = next(iter(node.items()))
+        if kind == "dict":
+            return {k: build(x) for k, x in v.items()}
+        if kind == "list":
+            return [build(x) for x in v]
+        if kind == "tensor":
+            return torch.from_numpy(g[v])
+        return g[v] if kind == "ndarray" else v
+
+    return build(json.loads(str(g["skeleton"])))
 
 
 def _same(a, b):
@@ -84,12 +90,11 @@ def _same(a, b):
     return a == b
 
 
-@pytest.mark.skipif(not has_reference(), reason="reference checkout not present")
 def test_collate_kitti_equals_reference_function():
     from det3d.torchie.parallel import collate_kitti
 
     batch = [_sample(i, n) for i, n in enumerate((7, 0, 13))]
-    want = _reference_collate()(batch)
+    want = _reference_collate_result()
     got = collate_kitti(batch)
     assert set(got) == set(want)
     for k in want:

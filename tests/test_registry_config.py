@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import REFERENCE, ROOT, has_reference, load_golden
+from conftest import ROOT, load_golden, reference_config
 
 
 def test_registry_semantics():
@@ -61,7 +61,6 @@ def test_shipped_config_builds_second():
     assert tuple(sd["neck.blocks.0.1.weight"].shape) == (128, 128, 3, 3)
 
 
-@pytest.mark.skipif(not has_reference(), reason="reference checkout not present")
 @pytest.mark.parametrize("rel", [
     "examples/second/configs/kitti_car_vfev3_spmiddlefhd_rpn1_mghead_syncbn.py",
     "examples/cbgs/configs/nusc_all_vfev3_spmiddleresnetfhd_rpn2_mghead_syncbn.py",
@@ -71,7 +70,7 @@ def test_reference_config_loads_unchanged(rel):
     from det3d.models import build_detector
     from det3d.torchie import Config
 
-    cfg = Config.fromfile(os.path.join(REFERENCE, rel))
+    cfg = reference_config(rel)
     model = build_detector(cfg.model, train_cfg=None, test_cfg=cfg.test_cfg)
     if "point_pillars" in rel:
         assert type(model).__name__ == "PointPillars"
